@@ -4,6 +4,7 @@ per other BASELINE configuration.
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm (numpy) on the host cores
+    python bench.py ... --dump-outputs DIR                   # also the records of the last timed step, DIR/<field>.npy
 
 One STEP = one pass of the hot path over one batch of synthetic input: `calls_per_step` x `blocks_per_call` independent
 1-ms IQ blocks @ 2.046 Msps (default 12 x 256 = 3072 blocks, 6.3 Msamples, ~25 ms of GPU work), each searched over the full
@@ -50,6 +51,21 @@ METRIC = "IQ Msamples/s through 32-PRN x 41-Doppler acquisition (1 ms non-cohere
 L2_BYTES = 126 << 20
 PLANTED = [(3, -3000.0, 5, 1.0, 0.3), (11, 4500.0, 1234, 2.0, 0.3), (25, 1500.0, 777, 0.3, 0.3), (32, -9500.0, 2045, 2.5, 0.3)]
 MAG_TOL = 1e-5  # DESIGN.md section 6
+DUMP_BYTES = 63_000_000  # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir: str, blocks: np.ndarray, records: dict) -> None:
+    """--dump-outputs: per-cell records of the last timed step as <field>.npy, each [blocks, 32 PRN, D Doppler] in float32 or
+    float64, plus block.npy, the index of each block in the IQ the step read.  The inputs are seeded, so two builds run with the
+    same arguments can be compared file for file; blocks beyond the size budget are dropped by a fixed, seeded choice."""
+    per_block = 8 + sum(a[0].nbytes for a in records.values())
+    keep = np.arange(len(blocks))
+    if per_block * len(blocks) > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(len(blocks), DUMP_BYTES // per_block, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "block.npy"), blocks[keep].astype(np.float64))
+    for name, a in records.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[keep])
 
 
 def alg_bytes(n: int, n_dop: int, m: int, n_blocks: int = 1) -> float:
@@ -263,7 +279,7 @@ def run_reference(args, rank: int, world: int) -> None:
     blocks = make_ring(nb * 2, seed=1)
     times = []
     for k in range(args.warmup + args.steps):
-        _, sec = pool.grid(blocks[(k % 2) * nb:(k % 2 + 1) * nb], FS, N, DOPPLERS)
+        ref, sec = pool.grid(blocks[(k % 2) * nb:(k % 2 + 1) * nb], FS, N, DOPPLERS)
         times.append(sec)
     pool.close()
     per_step = times[args.warmup:]
@@ -281,6 +297,9 @@ def run_reference(args, rank: int, world: int) -> None:
         "gpu_launches": 0, "wall_s": time.perf_counter() - t_start,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, (k % 2) * nb + np.arange(nb),
+                     {f: ref[..., i] for i, f in enumerate(("peak", "argmax", "sum", "count"))})
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -429,6 +448,14 @@ def run_ours(args, rank: int, local_rank: int, world: int) -> None:
     launches0 = eng.launch_count
     ms_total = g.timed(device_step, args.steps, first=args.warmup)
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        # the record ring has 4 slots: it still holds the last min(C, 4) calls of the last timed step
+        last = [(args.warmup + args.steps - 1) * C + c for c in range(max(0, C - 4), C)]
+        rec = np.concatenate([rec_dev[j % 4].cpu().numpy().view(_native.RECORD_DTYPE).reshape(B, N_PRN, len(DOPPLERS))
+                              for j in last])
+        dump_outputs(args.dump_outputs, np.concatenate([(j % n_slots) * B + np.arange(B) for j in last]),
+                     {"peak": rec["peak"], "argmax": rec["argmax"].astype(np.float32), "sum": rec["sum"],
+                      "count": rec["count"].astype(np.float32)})
     t_end = time.perf_counter() + 0.3  # continuation of the same loop so that short runs still get clock samples under load
     k = args.warmup + args.steps
     while time.perf_counter() < t_end:
@@ -1081,12 +1108,13 @@ def main() -> None:
     ap.add_argument("--cpu-blocks", type=int, default=4)
     ap.add_argument("--cpu-blocks-per-step", type=int, default=8)
     ap.add_argument("--no-configs", action="store_true", help="skip the config 3 / 4 / 5 sub-lines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's per-cell records of the last timed step to DIR/<field>.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
-        args.steps = min(args.steps, 500)  # bounded: ~50 ms per CPU step
         run_reference(args, rank, world)
     else:
         run_ours(args, rank, local_rank, world)

@@ -29,10 +29,12 @@ def emu_lib():
     """Host lane emulator (tests/emu): the product's lane-level device functions compiled for the CPU."""
     import ctypes
 
+    from gypsum_b200 import build
+
     src = os.path.join(ROOT, "tests", "emu", "emu.cu")
     out = os.path.join(ROOT, "tests", "emu", "libgbemu.so")
     deps = [src] + [os.path.join(ROOT, "gypsum_b200", "csrc", f) for f in ("warp_fft.cuh", "fft32_gen.cuh", "cplx2.cuh", "gb_common.cuh", "tracker_core.cuh", "bits_core.cuh")]
     if not os.path.exists(out) or any(os.path.getmtime(d) > os.path.getmtime(out) for d in deps):
-        subprocess.run(["nvcc", "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", out, src], check=True,
+        subprocess.run([build._nvcc(), "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", out, src], check=True,
                        capture_output=True)
     return ctypes.CDLL(out)

@@ -1,5 +1,6 @@
 """The oracle (oracle/gypsum_oracle.py) against fixtures produced by the live reference (tools/make_golden.py)
 and against the only known-answer table the reference holds (IS-GPS-200 first ten chips)."""
+import hashlib
 import os
 
 import numpy as np
@@ -50,8 +51,12 @@ def test_oracle_profiles_bit_exact_with_reference(name, n, n_ms, k):
     prn = o.replica(sv, n)
     nc = o.integrate(o.NON_COHERENT, x, fs, n, f, prn)
     co = o.integrate(o.COHERENT, x, fs, n, f, prn)
-    assert np.array_equal(nc, z[f"{name}__{k}__noncoherent"])
-    assert np.array_equal(co, z[f"{name}__{k}__coherent"])
+    # the recorded sample first (a failure shows the values), then the digest of every value
+    idx = z[f"{name}__{k}__sample_idx"]
+    assert np.array_equal(nc[idx], z[f"{name}__{k}__noncoherent_sample"])
+    assert np.array_equal(co[idx], z[f"{name}__{k}__coherent_sample"])
+    assert hashlib.sha256(nc.tobytes()).digest() == z[f"{name}__{k}__noncoherent_sha256"].tobytes()
+    assert hashlib.sha256(co.tobytes()).digest() == z[f"{name}__{k}__coherent_sha256"].tobytes()
     assert o.peak_strength(nc) == float(z[f"{name}__{k}__strength"])
 
 

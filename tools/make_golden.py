@@ -1,10 +1,11 @@
-"""Generate tests/golden/*.npz by running the LIVE reference (/root/reference) in the build container.
+"""Generate tests/golden/*.npz by running the LIVE reference (the original gypsum project).
 
 The reference has no golden vectors of its own (SURVEY.md F2), so parity is pinned on the reference's own
-outputs: this script imports gypsum.* from /root/reference (read-only, unmodified) and records what its
-functions return on seeded synthetic input.  Run:  python tools/make_golden.py
-The fixtures travel to the GPU box; /root/reference does not.
+outputs: this script imports gypsum.* from a checkout of the reference (read-only, unmodified) and records what
+its functions return on seeded synthetic input.  Run:  python tools/make_golden.py PATH_TO_REFERENCE_CHECKOUT
+The tests read only the fixtures; they never need the reference itself.
 """
+import hashlib
 import os
 import sys
 
@@ -12,7 +13,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+if len(sys.argv) != 2:
+    sys.exit("usage: python tools/make_golden.py PATH_TO_REFERENCE_CHECKOUT")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 
 from gypsum.acquisition import GpsSatelliteDetector  # noqa: E402
 from gypsum.antenna_sample_provider import SampleProviderAttributes  # noqa: E402
@@ -27,6 +30,11 @@ from gypsum.utils import (  # noqa: E402
 from oracle import gypsum_oracle as o  # noqa: E402  (only for synth_iq: identical input bytes everywhere)
 
 OUT = os.path.join(ROOT, "tests", "golden")
+PROFILE_SAMPLE = 64  # profile values stored per cell beside the digests; the peak index is always one of them
+
+
+def sha256(a: np.ndarray) -> np.ndarray:
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)
 
 
 class _Bytes(np.ndarray):
@@ -52,6 +60,8 @@ def main():
     )
 
     # ---- per-cell profiles (utils.py:77) at the three sample rates ----
+    # Whole profiles would exceed 1 MB, so each is kept as the SHA-256 of its bytes (the oracle's float64 profile must
+    # hash to it: bit-exact over every value) plus a seeded sample of values that shows the size of any difference.
     cases = {}
     for name, n, n_ms, planted, cells in [
         ("n2046_m1", 2046, 1, [(25, 1500.0, 777, 0.3, 0.5)], [(25, 1500), (25, -3500), (3, 0), (25, 1000.5)]),
@@ -71,8 +81,12 @@ def main():
                                                                 sat.prn_as_complex)
             cases[f"{name}__{k}__sv"] = np.int64(sv)
             cases[f"{name}__{k}__doppler"] = np.float64(f)
-            cases[f"{name}__{k}__noncoherent"] = nc
-            cases[f"{name}__{k}__coherent"] = co
+            idx = np.union1d(np.random.default_rng(k).choice(n, PROFILE_SAMPLE - 1, replace=False), [int(np.argmax(nc))])
+            cases[f"{name}__{k}__sample_idx"] = idx.astype(np.int64)
+            cases[f"{name}__{k}__noncoherent_sample"] = nc[idx]
+            cases[f"{name}__{k}__coherent_sample"] = co[idx]
+            cases[f"{name}__{k}__noncoherent_sha256"] = sha256(nc)
+            cases[f"{name}__{k}__coherent_sha256"] = sha256(co)
             cases[f"{name}__{k}__strength"] = np.float64(get_normalized_correlation_peak_strength(nc))
         cases[f"{name}__planted"] = np.array(planted, dtype=np.float64)
     np.savez_compressed(os.path.join(OUT, "cell_profiles.npz"), **cases)
