@@ -9,6 +9,8 @@
 #include <map>
 #include <numeric>
 #include <string>
+#include <tuple>
+#include <utility>
 #include <vector>
 
 #include "../../include/gypsum_b200.h"
@@ -23,46 +25,37 @@ namespace {
 
 thread_local std::string g_create_error;
 
-template <class T>
-struct DevBuf {
+// A growable allocation that frees itself.  The engine's device must be current when it is destroyed or grown.
+template <class T, cudaError_t (*Alloc)(void**, size_t), cudaError_t (*Free)(void*)>
+class Buf {
+public:
     T* p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(Buf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { release(); }
     cudaError_t ensure(size_t n) {
         if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        release();
         size_t want = std::max(n, static_cast<size_t>(16));
-        cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&p), want * sizeof(T));
+        cudaError_t e = Alloc(reinterpret_cast<void**>(&p), want * sizeof(T));
         if (e == cudaSuccess) cap = want;
         return e;
     }
+
+private:
     void release() {
-        if (p) cudaFree(p);
+        if (p) Free(p);
         p = nullptr;
         cap = 0;
     }
 };
 template <class T>
-struct PinnedBuf {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t ensure(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = std::max(n, static_cast<size_t>(16));
-        cudaError_t e = cudaMallocHost(reinterpret_cast<void**>(&p), want * sizeof(T));
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
+using DevBuf = Buf<T, cudaMalloc, cudaFree>;
+template <class T>
+using PinnedBuf = Buf<T, cudaMallocHost, cudaFreeHost>;
 
 int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
@@ -113,14 +106,23 @@ struct gb200_engine {
     PinnedBuf<BestRecord> h_best;
     // gb200_acquire_grid_host: one CUDA graph (copy-in, doppler_spectra, correlate_cells, copy-out) per grid shape
     struct HostGraph {
+        // What a captured graph bakes in: the grid's shape, every buffer its nodes dereference and the capture stream.
+        struct Key {
+            int n_blocks, M, P, D, kind;
+            const void *iq_dev, *rec_dev, *iq_stage, *rec_stage, *spec, *d_dop, *d_prn, *crep;
+            const void* rec_target;  // where the captured correlate kernel stores its records
+            cudaStream_t stream;
+            auto tie() const {
+                return std::tie(n_blocks, M, P, D, kind, iq_dev, rec_dev, iq_stage, rec_stage, spec, d_dop, d_prn, crep, rec_target,
+                                stream);
+            }
+            bool operator==(const Key& o) const { return tie() == o.tie(); }
+        };
         cudaGraphExec_t exec = nullptr;
-        int n_blocks = 0, M = 0, P = 0, D = 0, kind = 0, seen = 0;
-        std::vector<double> dop;
+        int seen = 0;
+        Key key{};
+        std::vector<double> dop;  // the grid's axes, compared in place against the caller's
         std::vector<int> prn;
-        const void *iq_dev = nullptr, *rec_dev = nullptr, *iq_stage = nullptr, *rec_stage = nullptr, *spec = nullptr;
-        const void *d_dop = nullptr, *d_prn = nullptr, *crep = nullptr;  // what the captured kernels dereference besides the above
-        const void* rec_target = nullptr;  // where the captured correlate kernel stores its records
-        cudaStream_t stream = nullptr;
     } hg;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[2];
     size_t ev_used[2] = {0, 0};
@@ -128,33 +130,6 @@ struct gb200_engine {
 
     ~gb200_engine() {
         if (hg.exec) cudaGraphExecDestroy(hg.exec);
-        d_best.release();
-        h_best.release();
-        tw1.release();
-        tw2.release();
-        crep.release();
-        d_replica.release();
-        iq_own.release();
-        spec.release();
-        chips.release();
-        d_doppler.release();
-        d_ints.release();
-        d_records.release();
-        d_profile.release();
-        r_state.release();
-        r_doppler.release();
-        r_records.release();
-        r_ints.release();
-        r_results.release();
-        r_cell_prn.release();
-        rh_cell_prn.release();
-        rh_ints.release();
-        rh_results.release();
-        h_iq.release();
-        h_records.release();
-        h_ints.release();
-        h_doubles.release();
-        h_profile.release();
         for (auto& pool : ev)
             for (auto& pr : pool) {
                 cudaEventDestroy(pr.first);
@@ -202,10 +177,18 @@ struct gb200_grid_stream {
         gb200_cell_record* out = nullptr;  // where this batch's records go
         bool staged_out = false;
         cudaEvent_t h2d = nullptr, done = nullptr, d2h = nullptr;
+        ~Slot() {
+            for (cudaEvent_t ev : {h2d, done, d2h})
+                if (ev) cudaEventDestroy(ev);
+        }
     };
     std::vector<Slot> slots;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     long long head = 0, tail = 0;  // batches submitted / collected
+    ~gb200_grid_stream() {
+        if (s_in) cudaStreamDestroy(s_in);
+        if (s_out) cudaStreamDestroy(s_out);
+    }
 };
 
 // Device-resident rolling window of the newest milliseconds; every millisecond is stored at slot k and at slot
@@ -239,6 +222,13 @@ static_assert(sizeof(gb200_bit_event) == sizeof(BitEvent), "ABI bit event and de
         }                                                                                                  \
     } while (0)
 
+// passes on the GB200_* code of a call that has already set the error message
+#define GB_TRY(expr)            \
+    do {                        \
+        const int rc_ = (expr); \
+        if (rc_) return rc_;    \
+    } while (0)
+
 namespace {
 
 // optional event bracket around one kernel launch (measurement aid, off by default)
@@ -263,14 +253,12 @@ struct TimedLaunch {
     }
 };
 
-int gcd_int(int a, int b) { return b ? gcd_int(b, a % b) : a; }
-
 // How many warp pairs share one cell.  With plenty of cells per pair each pair keeps a whole cell (no cross-pair
 // merge, no CTA-wide barrier); small launches split a cell's polyphase branches over pairs to fill the machine.
 int pick_rsplit(const gb200_engine* e, int np, long long n_cells) {
     if (e->rsplit_override > 0 && e->s % e->rsplit_override == 0 && np % e->rsplit_override == 0) return e->rsplit_override;
     if (n_cells >= 8LL * e->num_sms * np) return 1;
-    return gcd_int(e->s, np);
+    return std::gcd(e->s, np);
 }
 
 // Non-coherent, record-only launches use the one-warp-per-transform kernel: 12 warps per CTA (168 registers) for
@@ -291,15 +279,186 @@ int pick_np(const gb200_engine* e, int M, int kind, bool profile) {
     return (M == 1 && kind == GB200_NON_COHERENT && !profile) ? 10 : 8;
 }
 
+// The correlate kernel of one launch shape: nw warps per CTA of the one-warp kernel, or (nw = 0) the pair kernel with np pairs;
+// rsplit slots share a cell, so a group holds cpg cells.
+struct CorrPlan {
+    int nw, np, rsplit, cpg;
+};
+
+CorrPlan plan_correlate(const gb200_engine* e, int M, int kind, bool profile, long long n_cells) {
+    const int nw = pick_w2048(e, M, kind, profile);
+    const int np = nw ? nw : pick_np(e, M, kind, profile);  // CTA "slots": warps (one-warp kernel) or warp pairs
+    const int rsplit = pick_rsplit(e, np, n_cells);
+    return {nw, np, rsplit, np / rsplit};
+}
+
 size_t unit_floats2(const gb200_engine* e, int M) { return static_cast<size_t>(M) * e->s * 2 * kFft; }
 
-int check_common(gb200_engine* e, int n_ms, int kind) {
+// need_replicas = false: the caller brings its own replica (gb200_correlation_profile_replica)
+int check_common(gb200_engine* e, int n_ms, int kind, bool need_replicas = true) {
     if (!e) return GB200_EINVAL;
     if (kind != GB200_COHERENT && kind != GB200_NON_COHERENT) GB_FAIL(e, GB200_EINVAL, "Unexpected integration type");
-    if (e->n_prn == 0) GB_FAIL(e, GB200_ESTATE, "no PRN replicas loaded (gb200_set_replicas)");
+    if (need_replicas && e->n_prn == 0) GB_FAIL(e, GB200_ESTATE, "no PRN replicas loaded (gb200_set_replicas)");
     if (!e->iq) GB_FAIL(e, GB200_ESTATE, "no IQ loaded (gb200_upload_iq / gb200_bind_iq_device)");
     if (n_ms < 1) GB_FAIL(e, GB200_EINVAL, "need at least one whole millisecond of samples");
     return GB200_OK;
+}
+
+int check_prns(gb200_engine* e, const int32_t* prn_idx, int n) {
+    for (int i = 0; i < n; ++i)
+        if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
+    return GB200_OK;
+}
+
+// n_ms milliseconds from the start of the bound IQ
+int check_samples(gb200_engine* e, int n_ms) {
+    const long long need = static_cast<long long>(n_ms) * e->N;
+    if (need > e->iq_samples)
+        GB_FAIL(e, GB200_EINVAL, "need %lld samples, %lld loaded", need, static_cast<long long>(e->iq_samples));
+    return GB200_OK;
+}
+
+int check_channel(gb200_tracker* t, int channel) {
+    if (channel < 0 || channel >= t->n_channels) GB_FAIL(t->e, GB200_EINVAL, "channel %d out of range", channel);
+    return GB200_OK;
+}
+
+// A device buffer and its pinned host staging, both grown to at least n elements.
+template <class T>
+cudaError_t ensure_staging(DevBuf<T>& dev, PinnedBuf<T>& host, size_t n) {
+    const cudaError_t ce = dev.ensure(n);
+    return ce == cudaSuccess ? host.ensure(n) : ce;
+}
+
+// The staging pair (device buffer, pinned host buffer) receives n elements of src and queues their upload.  The caller makes
+// sure the host buffer is no longer in flight.
+template <class T>
+int stage_upload(gb200_engine* e, DevBuf<T>& dev, PinnedBuf<T>& host, const T* src, size_t n) {
+    GB_CUDA(e, ensure_staging(dev, host, n));
+    memcpy(host.p, src, sizeof(T) * n);
+    GB_CUDA(e, cudaMemcpyAsync(dev.p, host.p, sizeof(T) * n, cudaMemcpyHostToDevice, e->stream));
+    return GB200_OK;
+}
+
+// n elements from the device to the caller through pinned staging (already large enough): one copy, one synchronise.
+template <class T>
+int download(gb200_engine* e, void* out_host, PinnedBuf<T>& stage, const T* src_dev, size_t n) {
+    GB_CUDA(e, cudaMemcpyAsync(stage.p, src_dev, n * sizeof(T), cudaMemcpyDeviceToHost, e->stream));
+    GB_CUDA(e, cudaStreamSynchronize(e->stream));
+    memcpy(out_host, stage.p, n * sizeof(T));
+    return GB200_OK;
+}
+
+// The device address of page-locked host memory, or null when p is pageable.
+void* pinned_alias(const void* p) {
+    cudaPointerAttributes attr{};
+    const bool pinned = cudaPointerGetAttributes(&attr, p) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    return pinned ? attr.devicePointer : nullptr;
+}
+
+// Where a copy of n samples from the caller's buffer starts: the buffer itself when it is pinned, else the pinned staging
+// buffer, refilled once the stream has stopped reading it.
+int pinned_source(gb200_engine* e, PinnedBuf<float2>& stage, const float* host, size_t n, const float2** src) {
+    *src = reinterpret_cast<const float2*>(host);
+    if (pinned_alias(host)) return GB200_OK;
+    GB_CUDA(e, cudaStreamSynchronize(e->stream));
+    GB_CUDA(e, stage.ensure(std::max<size_t>(n, 1)));
+    memcpy(stage.p, host, n * sizeof(float2));
+    *src = stage.p;
+    return GB200_OK;
+}
+
+cudaError_t ensure_fused_configured(gb200_engine* e) {
+    if (e->fused_configured) return cudaSuccess;
+    const cudaError_t ce = configure_fused_kernel();
+    e->fused_configured = ce == cudaSuccess;
+    return ce;
+}
+
+// The three acquisition kernels, each with its optional timing events and counted in e->launches.
+int enqueue_spectra(gb200_engine* e, const float2* iq, long long block_stride, const double* dop, int M, int n_doppler,
+                    int n_units) {
+    SpectraArgs sa{};
+    sa.iq = iq;
+    sa.doppler = dop;
+    sa.spec = e->spec.p;
+    sa.tw1 = e->tw1.p;
+    sa.tw2 = e->tw2.p;
+    sa.block_stride = block_stride;
+    sa.inv_fs = 1.0 / static_cast<double>(e->fs);
+    sa.N = e->N;
+    sa.s = e->s;
+    sa.M = M;
+    sa.n_doppler = n_doppler;
+    sa.n_units = n_units;
+    TimedLaunch tl(e, 0);
+    GB_CUDA(e, launch_doppler_spectra(sa, e->stream));
+    e->launches++;
+    return GB200_OK;
+}
+
+// The engine's part of a correlate launch; the caller adds the grid-mode or list-mode cell layout.
+CorrelateArgs correlate_args(const gb200_engine* e, int M, int kind, CellRecord* records) {
+    CorrelateArgs ca{};
+    ca.spec = e->spec.p;
+    ca.crep = e->crep.p;
+    ca.tw1 = e->tw1.p;
+    ca.tw2 = e->tw2.p;
+    ca.records = records;
+    ca.N = e->N;
+    ca.s = e->s;
+    ca.M = M;
+    ca.kind = kind;
+    return ca;
+}
+
+int enqueue_correlate(gb200_engine* e, const CorrPlan& plan, CorrelateArgs ca, int grid) {
+    ca.rsplit = plan.rsplit;
+    TimedLaunch tl(e, 1);
+    if (plan.nw) GB_CUDA(e, launch_correlate_w2048(ca, plan.nw, grid, e->stream));
+    else GB_CUDA(e, launch_correlate_cells(ca, plan.np, grid, e->stream));
+    e->launches++;
+    return GB200_OK;
+}
+
+// one CTA per cell, whole pipeline in one kernel
+int enqueue_fused(gb200_engine* e, int M, int kind, const double* dop, const int* prn, const int* probe, CellRecord* records,
+                  int n_cells) {
+    FusedArgs fa{};
+    fa.iq = e->iq;
+    fa.doppler = dop;
+    fa.prn = prn;
+    fa.probe = probe;
+    fa.records = records;
+    fa.crep = e->crep.p;
+    fa.tw1 = e->tw1.p;
+    fa.tw2 = e->tw2.p;
+    fa.inv_fs = 1.0 / static_cast<double>(e->fs);
+    fa.N = e->N;
+    fa.M = M;
+    fa.n_cells = n_cells;
+    TimedLaunch tl(e, 1);
+    GB_CUDA(e, launch_acquire_fused(fa, e->s, kind, e->stream));
+    e->launches++;
+    return GB200_OK;
+}
+
+// L2 windows of the one-warp kernel (see the kernel): a batch whose spectra exceed L2 is walked in equal runs of units of
+// about GB200_L2_WINDOW_MB (default 40; 0 = off), as long as a window still gives every CTA at least two groups (config 5's
+// heavy cells: 2.8 groups per CTA and window; the kernel's round-robin of the extra groups keeps the CTAs together).
+// Returns the chunks per window, 0 for one window over the whole batch.
+int l2_window_chunks(size_t batch_bytes, int chunks, int P, int grid) {
+    static const size_t win_bytes = static_cast<size_t>(std::max(0, env_int("GB200_L2_WINDOW_MB", 40))) << 20;
+    if (!win_bytes || batch_bytes <= win_bytes + win_bytes / 2) return 0;
+    const long long n_win = static_cast<long long>((batch_bytes + win_bytes - 1) / win_bytes);
+    long long wc = (chunks + n_win - 1) / n_win;
+    // a window whose P * wc groups divide evenly among the CTAs, when one exists within a quarter of the target size
+    const long long q = grid / std::gcd(P, grid);
+    const long long even = ((wc + q / 2) / q) * q;
+    if (even > 0 && even * 4 >= wc * 3 && even * 4 <= wc * 5) wc = even;
+    static const int min_groups = env_int("GB200_L2_WINDOW_MIN_GROUPS", 2);
+    return (wc * P >= static_cast<long long>(min_groups) * grid && wc < chunks) ? static_cast<int>(wc) : 0;
 }
 
 // The grid's axes (PRN rows in d_ints, Doppler bins in d_doppler) are uploaded only when they changed -- or when a list-mode
@@ -311,14 +470,9 @@ int upload_grid_axes(gb200_engine* e, const int32_t* prn_idx, int P, const doubl
                       memcmp(e->prn_cache.data(), prn_idx, sizeof(int) * P) == 0;
     if (same) return GB200_OK;
     GB_CUDA(e, cudaStreamSynchronize(e->stream));  // staging buffers may still be in flight
-    GB_CUDA(e, e->d_doppler.ensure(D));
-    GB_CUDA(e, e->d_ints.ensure(P));
-    GB_CUDA(e, e->h_doubles.ensure(D));
-    GB_CUDA(e, e->h_ints.ensure(P));
-    memcpy(e->h_doubles.p, dop, sizeof(double) * D);
-    memcpy(e->h_ints.p, prn_idx, sizeof(int) * P);
-    GB_CUDA(e, cudaMemcpyAsync(e->d_doppler.p, e->h_doubles.p, sizeof(double) * D, cudaMemcpyHostToDevice, e->stream));
-    GB_CUDA(e, cudaMemcpyAsync(e->d_ints.p, e->h_ints.p, sizeof(int) * P, cudaMemcpyHostToDevice, e->stream));
+    e->grid_cache_valid = false;                   // until both axes are queued
+    GB_TRY(stage_upload(e, e->d_doppler, e->h_doubles, dop, D));
+    GB_TRY(stage_upload(e, e->d_ints, e->h_ints, prn_idx, P));
     e->doppler_cache.assign(dop, dop + D);
     e->prn_cache.assign(prn_idx, prn_idx + P);
     e->grid_cache_valid = true;
@@ -328,17 +482,14 @@ int upload_grid_axes(gb200_engine* e, const int32_t* prn_idx, int P, const doubl
 // grid mode: all cells of n_blocks x prn list x doppler list; records written to rec_dev (device)
 int run_grid(gb200_engine* e, int n_blocks, int M, const int32_t* prn_idx, int P, const double* dop, int D, int kind,
              CellRecord* rec_dev) {
-    int rc = check_common(e, M, kind);
-    if (rc) return rc;
+    GB_TRY(check_common(e, M, kind));
     if (n_blocks < 1 || P < 1 || D < 1 || !prn_idx || !dop) GB_FAIL(e, GB200_EINVAL, "empty grid");
     if (static_cast<int64_t>(n_blocks) * M * e->N > e->iq_samples)
         GB_FAIL(e, GB200_EINVAL, "grid needs %lld samples, %lld loaded", static_cast<long long>(n_blocks) * M * e->N,
                 static_cast<long long>(e->iq_samples));
-    for (int i = 0; i < P; ++i)
-        if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
+    GB_TRY(check_prns(e, prn_idx, P));
 
-    rc = upload_grid_axes(e, prn_idx, P, dop, D);
-    if (rc) return rc;
+    GB_TRY(upload_grid_axes(e, prn_idx, P, dop, D));
 
     const size_t unit = unit_floats2(e, M);
     const size_t per_block = unit * D;
@@ -346,44 +497,14 @@ int run_grid(gb200_engine* e, int n_blocks, int M, const int32_t* prn_idx, int P
     nb = std::min(nb, n_blocks);
     GB_CUDA(e, e->spec.ensure(per_block * nb));
 
-    const int nw = pick_w2048(e, M, kind, false);
-    const int np = nw ? nw : pick_np(e, M, kind, false);  // CTA "slots": warps (one-warp kernel) or warp pairs
-    const int rsplit = pick_rsplit(e, np, static_cast<long long>(nb) * P * D);
-    const int cpg = np / rsplit;
+    const CorrPlan plan = plan_correlate(e, M, kind, false, static_cast<long long>(nb) * P * D);
     for (int b0 = 0; b0 < n_blocks; b0 += nb) {
         const int nbb = std::min(nb, n_blocks - b0);
-        const int chunks = (nbb * D + cpg - 1) / cpg;  // groups per PRN: its nbb*D cells in chunks of cpg
-        SpectraArgs sa{};
-        sa.iq = e->iq + static_cast<size_t>(b0) * M * e->N;
-        sa.doppler = e->d_doppler.p;
-        sa.spec = e->spec.p;
-        sa.tw1 = e->tw1.p;
-        sa.tw2 = e->tw2.p;
-        sa.block_stride = static_cast<long long>(M) * e->N;
-        sa.inv_fs = 1.0 / static_cast<double>(e->fs);
-        sa.N = e->N;
-        sa.s = e->s;
-        sa.M = M;
-        sa.n_doppler = D;
-        sa.n_units = nbb * D;
-        {
-            TimedLaunch tl(e, 0);
-            GB_CUDA(e, launch_doppler_spectra(sa, e->stream));
-        }
-        e->launches++;
+        const int chunks = (nbb * D + plan.cpg - 1) / plan.cpg;  // groups per PRN: its nbb*D cells in chunks of cpg
+        const long long stride = static_cast<long long>(M) * e->N;
+        GB_TRY(enqueue_spectra(e, e->iq + static_cast<size_t>(b0) * stride, stride, e->d_doppler.p, M, D, nbb * D));
 
-        CorrelateArgs ca{};
-        ca.spec = e->spec.p;
-        ca.crep = e->crep.p;
-        ca.tw1 = e->tw1.p;
-        ca.tw2 = e->tw2.p;
-        ca.records = rec_dev + static_cast<size_t>(b0) * P * D;
-        ca.profile = nullptr;
-        ca.N = e->N;
-        ca.s = e->s;
-        ca.M = M;
-        ca.kind = kind;
-        ca.rsplit = rsplit;
+        CorrelateArgs ca = correlate_args(e, M, kind, rec_dev + static_cast<size_t>(b0) * P * D);
         ca.n_groups = P * chunks;
         ca.grid_mode = 1;
         ca.P = P;
@@ -391,36 +512,9 @@ int run_grid(gb200_engine* e, int n_blocks, int M, const int32_t* prn_idx, int P
         ca.n_blocks = nbb;
         ca.chunks = chunks;
         ca.prn_idx = e->d_ints.p;
-        ca.cell_probe = nullptr;
         const int grid = std::min(ca.n_groups, e->num_sms);
-        // L2 windows of the one-warp kernel (see the kernel): a batch whose spectra exceed L2 is walked in equal runs of units of
-        // about GB200_L2_WINDOW_MB (default 40; 0 = off), as long as a window still gives every CTA at least two groups (config 5's
-        // heavy cells: 2.8 groups per CTA and window; the kernel's round-robin of the extra groups keeps the CTAs together).
-        static const size_t win_bytes = static_cast<size_t>(std::max(0, env_int("GB200_L2_WINDOW_MB", 40))) << 20;
-        ca.win_chunks = 0;
-        const size_t batch_bytes = static_cast<size_t>(nbb) * per_block * sizeof(float2);
-        if (nw && win_bytes && batch_bytes > win_bytes + win_bytes / 2) {
-            const long long n_win = static_cast<long long>((batch_bytes + win_bytes - 1) / win_bytes);
-            long long wc = (chunks + n_win - 1) / n_win;
-            // a window whose P * wc groups divide evenly among the CTAs, when one exists within a quarter of the target size
-            long long q = grid, gcd_a = P, gcd_b = grid;
-            while (gcd_b) {
-                const long long t = gcd_a % gcd_b;
-                gcd_a = gcd_b;
-                gcd_b = t;
-            }
-            q = grid / gcd_a;
-            const long long even = ((wc + q / 2) / q) * q;
-            if (even > 0 && even * 4 >= wc * 3 && even * 4 <= wc * 5) wc = even;
-            static const int min_groups = env_int("GB200_L2_WINDOW_MIN_GROUPS", 2);
-            if (wc * P >= static_cast<long long>(min_groups) * grid && wc < chunks) ca.win_chunks = static_cast<int>(wc);
-        }
-        {
-            TimedLaunch tl(e, 1);
-            if (nw) GB_CUDA(e, launch_correlate_w2048(ca, nw, grid, e->stream));
-            else GB_CUDA(e, launch_correlate_cells(ca, np, grid, e->stream));
-        }
-        e->launches++;
+        if (plan.nw) ca.win_chunks = l2_window_chunks(static_cast<size_t>(nbb) * per_block * sizeof(float2), chunks, P, grid);
+        GB_TRY(enqueue_correlate(e, plan, ca, grid));
     }
     return GB200_OK;
 }
@@ -428,14 +522,10 @@ int run_grid(gb200_engine* e, int n_blocks, int M, const int32_t* prn_idx, int P
 // list mode.  Cells are sorted by PRN and cut into chunks whose spectra fit the scratch budget.
 int run_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, const double* dop, const int32_t* probe, int M,
               int kind, CellRecord* rec_dev, float* profile_dev) {
-    int rc = check_common(e, M, kind);
-    if (rc) return rc;
+    GB_TRY(check_common(e, M, kind));
     if (n_cells < 1 || !prn_idx || !dop) GB_FAIL(e, GB200_EINVAL, "empty cell list");
-    if (static_cast<int64_t>(M) * e->N > e->iq_samples)
-        GB_FAIL(e, GB200_EINVAL, "need %lld samples, %lld loaded", static_cast<long long>(M) * e->N,
-                static_cast<long long>(e->iq_samples));
-    for (int i = 0; i < n_cells; ++i)
-        if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
+    GB_TRY(check_samples(e, M));
+    GB_TRY(check_prns(e, prn_idx, n_cells));
     e->grid_cache_valid = false;  // d_ints / d_doppler are about to be overwritten
 
     bool use_fused = e->fused == 1;
@@ -449,16 +539,10 @@ int run_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, const double
         use_fused = n_unique * 4 > n_cells || static_cast<long long>(n_cells) * M <= 8192;
     }
     if (use_fused && fused_supports(e->s) && !profile_dev) {
-        if (!e->fused_configured) {
-            GB_CUDA(e, configure_fused_kernel());
-            e->fused_configured = true;
-        }
-        // one CTA per cell, whole pipeline in one kernel
+        GB_CUDA(e, ensure_fused_configured(e));
         GB_CUDA(e, cudaStreamSynchronize(e->stream));
-        GB_CUDA(e, e->d_ints.ensure(static_cast<size_t>(n_cells) * 2));
-        GB_CUDA(e, e->h_ints.ensure(static_cast<size_t>(n_cells) * 2));
-        GB_CUDA(e, e->d_doppler.ensure(n_cells));
-        GB_CUDA(e, e->h_doubles.ensure(n_cells));
+        GB_CUDA(e, ensure_staging(e->d_ints, e->h_ints, static_cast<size_t>(n_cells) * 2));
+        GB_CUDA(e, ensure_staging(e->d_doppler, e->h_doubles, n_cells));
         for (int i = 0; i < n_cells; ++i) {
             e->h_ints.p[i] = prn_idx[i];
             e->h_ints.p[n_cells + i] = probe ? probe[i] : -1;
@@ -466,31 +550,11 @@ int run_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, const double
         }
         GB_CUDA(e, cudaMemcpyAsync(e->d_ints.p, e->h_ints.p, sizeof(int) * 2 * n_cells, cudaMemcpyHostToDevice, e->stream));
         GB_CUDA(e, cudaMemcpyAsync(e->d_doppler.p, e->h_doubles.p, sizeof(double) * n_cells, cudaMemcpyHostToDevice, e->stream));
-        FusedArgs fa{};
-        fa.iq = e->iq;
-        fa.doppler = e->d_doppler.p;
-        fa.prn = e->d_ints.p;
-        fa.probe = e->d_ints.p + n_cells;
-        fa.records = rec_dev;
-        fa.crep = e->crep.p;
-        fa.tw1 = e->tw1.p;
-        fa.tw2 = e->tw2.p;
-        fa.inv_fs = 1.0 / static_cast<double>(e->fs);
-        fa.N = e->N;
-        fa.M = M;
-        fa.n_cells = n_cells;
-        {
-            TimedLaunch tl(e, 1);
-            GB_CUDA(e, launch_acquire_fused(fa, e->s, kind, e->stream));
-        }
-        e->launches++;
-        return GB200_OK;
+        return enqueue_fused(e, M, kind, e->d_doppler.p, e->d_ints.p, e->d_ints.p + n_cells, rec_dev, n_cells);
     }
 
-    const int nw = pick_w2048(e, M, kind, profile_dev != nullptr);
-    const int np = nw ? nw : pick_np(e, M, kind, profile_dev != nullptr);
-    const int rsplit = pick_rsplit(e, np, n_cells);
-    const int cpg = np / rsplit;
+    const CorrPlan plan = plan_correlate(e, M, kind, profile_dev != nullptr, n_cells);
+    const int cpg = plan.cpg;
     std::vector<int> order(n_cells);
     std::iota(order.begin(), order.end(), 0);
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return prn_idx[a] < prn_idx[b]; });
@@ -501,10 +565,8 @@ int run_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, const double
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
     // probe indices live at the front of the int buffer for the whole call
     const size_t ints_needed = static_cast<size_t>(n_cells) * 3 + 3 * (static_cast<size_t>(n_cells) + 1);
-    GB_CUDA(e, e->d_ints.ensure(ints_needed));
-    GB_CUDA(e, e->h_ints.ensure(ints_needed));
-    GB_CUDA(e, e->d_doppler.ensure(n_cells));
-    GB_CUDA(e, e->h_doubles.ensure(n_cells));
+    GB_CUDA(e, ensure_staging(e->d_ints, e->h_ints, ints_needed));
+    GB_CUDA(e, ensure_staging(e->d_doppler, e->h_doubles, n_cells));
     for (int i = 0; i < n_cells; ++i) e->h_ints.p[i] = probe ? probe[i] : -1;
     GB_CUDA(e, cudaMemcpyAsync(e->d_ints.p, e->h_ints.p, sizeof(int) * n_cells, cudaMemcpyHostToDevice, e->stream));
     GB_CUDA(e, e->spec.ensure(unit * std::min(max_cells, n_cells)));
@@ -552,76 +614,32 @@ int run_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, const double
         GB_CUDA(e, cudaMemcpyAsync(di, hi, sizeof(int) * (2 * nc + 3 * ng), cudaMemcpyHostToDevice, e->stream));
         GB_CUDA(e, cudaMemcpyAsync(e->d_doppler.p, e->h_doubles.p, sizeof(double) * nu, cudaMemcpyHostToDevice, e->stream));
 
-        SpectraArgs sa{};
-        sa.iq = e->iq;
-        sa.doppler = e->d_doppler.p;
-        sa.spec = e->spec.p;
-        sa.tw1 = e->tw1.p;
-        sa.tw2 = e->tw2.p;
-        sa.block_stride = 0;
-        sa.inv_fs = 1.0 / static_cast<double>(e->fs);
-        sa.N = e->N;
-        sa.s = e->s;
-        sa.M = M;
-        sa.n_doppler = nu;
-        sa.n_units = nu;
-        {
-            TimedLaunch tl(e, 0);
-            GB_CUDA(e, launch_doppler_spectra(sa, e->stream));
-        }
-        e->launches++;
+        GB_TRY(enqueue_spectra(e, e->iq, 0, e->d_doppler.p, M, nu, nu));
 
-        CorrelateArgs ca{};
-        ca.spec = e->spec.p;
-        ca.crep = e->crep.p;
-        ca.tw1 = e->tw1.p;
-        ca.tw2 = e->tw2.p;
-        ca.records = rec_dev;
+        CorrelateArgs ca = correlate_args(e, M, kind, rec_dev);
         ca.profile = profile_dev;
-        ca.N = e->N;
-        ca.s = e->s;
-        ca.M = M;
-        ca.kind = kind;
-        ca.rsplit = rsplit;
         ca.n_groups = ng;
-        ca.grid_mode = 0;
         ca.cell_u = di;
         ca.cell_out = di + nc;
         ca.grp_first = di + 2 * nc;
         ca.grp_count = di + 2 * nc + ng;
         ca.grp_prn = di + 2 * nc + 2 * ng;
         ca.cell_probe = e->d_ints.p;
-        const int grid = std::min(ng, e->num_sms);
-        {
-            TimedLaunch tl(e, 1);
-            if (nw) GB_CUDA(e, launch_correlate_w2048(ca, nw, grid, e->stream));
-            else GB_CUDA(e, launch_correlate_cells(ca, np, grid, e->stream));
-        }
-        e->launches++;
+        GB_TRY(enqueue_correlate(e, plan, ca, std::min(ng, e->num_sms)));
         c0 = c1;
     }
     return GB200_OK;
 }
 
-bool is_pinned_host(const void* p) {
-    cudaPointerAttributes attr;
-    const bool pinned = cudaPointerGetAttributes(&attr, p) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-    cudaGetLastError();
-    return pinned;
-}
-
 // Records to the caller: straight DMA when the caller's buffer is pinned, else through the engine's pinned staging.
 int fetch_records(gb200_engine* e, size_t n, gb200_cell_record* out_host) {
-    if (is_pinned_host(out_host)) {
+    if (pinned_alias(out_host)) {
         GB_CUDA(e, cudaMemcpyAsync(out_host, e->d_records.p, n * sizeof(CellRecord), cudaMemcpyDeviceToHost, e->stream));
         GB_CUDA(e, cudaStreamSynchronize(e->stream));
         return GB200_OK;
     }
     GB_CUDA(e, e->h_records.ensure(n));
-    GB_CUDA(e, cudaMemcpyAsync(e->h_records.p, e->d_records.p, n * sizeof(CellRecord), cudaMemcpyDeviceToHost, e->stream));
-    GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->h_records.p, n * sizeof(CellRecord));
-    return GB200_OK;
+    return download(e, out_host, e->h_records, e->d_records.p, n);
 }
 
 }  // namespace
@@ -730,14 +748,8 @@ int gb200_upload_iq(gb200_engine* e, const float* iq_host, int64_t n_samples) {
     if (!iq_host || n_samples < 0) GB_FAIL(e, GB200_EINVAL, "bad IQ buffer");
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, e->iq_own.ensure(static_cast<size_t>(std::max<int64_t>(n_samples, 1))));
-    const void* src = iq_host;
-    const bool pinned = is_pinned_host(iq_host);
-    if (!pinned) {
-        GB_CUDA(e, cudaStreamSynchronize(e->stream));  // staging buffer may still be in flight
-        GB_CUDA(e, e->h_iq.ensure(static_cast<size_t>(std::max<int64_t>(n_samples, 1))));
-        memcpy(e->h_iq.p, iq_host, static_cast<size_t>(n_samples) * sizeof(float2));
-        src = e->h_iq.p;
-    }
+    const float2* src = nullptr;
+    GB_TRY(pinned_source(e, e->h_iq, iq_host, static_cast<size_t>(n_samples), &src));
     GB_CUDA(e, cudaMemcpyAsync(e->iq_own.p, src, static_cast<size_t>(n_samples) * sizeof(float2), cudaMemcpyHostToDevice,
                                e->stream));
     e->iq = e->iq_own.p;
@@ -771,8 +783,7 @@ int gb200_acquire_grid(gb200_engine* e, int n_blocks, int M, const int32_t* prn_
     if (n_blocks < 1 || P < 1 || D < 1) GB_FAIL(e, GB200_EINVAL, "empty grid");
     const size_t n = static_cast<size_t>(n_blocks) * P * D;
     GB_CUDA(e, e->d_records.ensure(n));
-    int rc = run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_records.p);
-    if (rc) return rc;
+    GB_TRY(run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_records.p));
     return fetch_records(e, n, out_host);
 }
 
@@ -785,8 +796,7 @@ int gb200_acquire_grid_best_device(gb200_engine* e, int n_blocks, int M, const i
     if (n_blocks < 1 || P < 1 || D < 1) GB_FAIL(e, GB200_EINVAL, "empty grid");
     const size_t n = static_cast<size_t>(n_blocks) * P * D;
     GB_CUDA(e, e->d_records.ensure(n));
-    int rc = run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_records.p);
-    if (rc) return rc;
+    GB_TRY(run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_records.p));
     GB_CUDA(e, launch_best_bins(n_blocks * P, D, e->N, e->d_records.p, e->d_doppler.p, static_cast<BestRecord*>(out_device),
                                 e->stream));
     e->launches++;
@@ -801,14 +811,9 @@ int gb200_acquire_grid_best(gb200_engine* e, int n_blocks, int M, const int32_t*
     if (n_blocks < 1 || P < 1 || D < 1) GB_FAIL(e, GB200_EINVAL, "empty grid");
     const size_t n = static_cast<size_t>(n_blocks) * P;
     GB_CUDA(e, cudaStreamSynchronize(e->stream));  // h_best may still be in flight
-    GB_CUDA(e, e->d_best.ensure(n));
-    GB_CUDA(e, e->h_best.ensure(n));
-    int rc = gb200_acquire_grid_best_device(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_best.p);
-    if (rc) return rc;
-    GB_CUDA(e, cudaMemcpyAsync(e->h_best.p, e->d_best.p, n * sizeof(BestRecord), cudaMemcpyDeviceToHost, e->stream));
-    GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->h_best.p, n * sizeof(BestRecord));
-    return GB200_OK;
+    GB_CUDA(e, ensure_staging(e->d_best, e->h_best, n));
+    GB_TRY(gb200_acquire_grid_best_device(e, n_blocks, M, prn_idx, P, dop, D, kind, e->d_best.p));
+    return download(e, out_host, e->h_best, e->d_best.p, n);
 }
 
 // Host to host in one call.  The first call of a shape runs eagerly (it may have to upload the axes and grow buffers,
@@ -824,29 +829,17 @@ int gb200_acquire_grid_host(gb200_engine* e, const float* iq_host, int n_blocks,
     const size_t spec_bytes = unit_floats2(e, M) * D * sizeof(float2) * n_blocks;
     static const bool graphs = env_int("GB200_GRAPH", 1) != 0;
     if (!graphs || e->timing || spec_bytes > e->spec_budget_bytes) {  // several scratch batches / per-kernel events: plain path
-        int rc = gb200_upload_iq(e, iq_host, static_cast<int64_t>(n_iq));
-        if (rc) return rc;
+        GB_TRY(gb200_upload_iq(e, iq_host, static_cast<int64_t>(n_iq)));
         return gb200_acquire_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, out_host);
     }
     GB_CUDA(e, cudaStreamSynchronize(e->stream));  // the pinned staging buffers may still be in flight
-    GB_CUDA(e, e->iq_own.ensure(n_iq));
-    GB_CUDA(e, e->h_iq.ensure(n_iq));
-    GB_CUDA(e, e->d_records.ensure(n_rec));
-    GB_CUDA(e, e->h_records.ensure(n_rec));
+    GB_CUDA(e, ensure_staging(e->iq_own, e->h_iq, n_iq));
+    GB_CUDA(e, ensure_staging(e->d_records, e->h_records, n_rec));
     // Large pinned inputs (a 10-ms window is 327 KB) are copied by the DMA engine straight from the caller's buffer: staging them
     // would cost a 15-20 us host memcpy.  The copy node of the graph has its source baked in, so those calls launch eagerly
     // (1.7 us more than a replay on this host, profiles/launch_latency_r2.log).  Small inputs are staged and replayed.
-    const float2* h2d_src = e->h_iq.p;
-    bool eager_src = false;
-    if (n_iq * sizeof(float2) > (64u << 10)) {
-        cudaPointerAttributes pa{};
-        if (cudaPointerGetAttributes(&pa, iq_host) == cudaSuccess && pa.type == cudaMemoryTypeHost) {
-            h2d_src = reinterpret_cast<const float2*>(iq_host);
-            eager_src = true;
-        } else {
-            cudaGetLastError();
-        }
-    }
+    const bool eager_src = n_iq * sizeof(float2) > (64u << 10) && pinned_alias(iq_host);
+    const float2* h2d_src = eager_src ? reinterpret_cast<const float2*>(iq_host) : e->h_iq.p;
     if (!eager_src) memcpy(e->h_iq.p, iq_host, n_iq * sizeof(float2));
     e->iq = e->iq_own.p;
     e->iq_samples = static_cast<int64_t>(n_iq);
@@ -856,44 +849,32 @@ int gb200_acquire_grid_host(gb200_engine* e, const float* iq_host, int n_blocks,
     // moved buffer (gb200_set_replicas with a larger table, a larger list-mode call) as a new shape.
     {
         if (e->n_prn == 0) GB_FAIL(e, GB200_ESTATE, "no PRN replicas loaded (gb200_set_replicas)");
-        for (int i = 0; i < P; ++i)
-            if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
-        int rc = upload_grid_axes(e, prn_idx, P, dop, D);
-        if (rc) return rc;
+        GB_TRY(check_prns(e, prn_idx, P));
+        GB_TRY(upload_grid_axes(e, prn_idx, P, dop, D));
     }
     // Small grids: the correlate kernel stores its 32-byte records straight into pinned (device-mapped under UVA) memory --
     // posted PCIe writes at the kernel's tail instead of a separate copy node behind it -- and into the CALLER's buffer when that
     // is itself pinned, which also saves the host copy out of the staging buffer.
     const bool direct = n_rec * sizeof(CellRecord) <= (256u << 10);
-    CellRecord* rec_target = direct ? e->h_records.p : e->d_records.p;
-    bool to_caller = false;
-    if (direct) {
-        cudaPointerAttributes pa{};
-        if (cudaPointerGetAttributes(&pa, out_host) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.devicePointer) {
-            rec_target = static_cast<CellRecord*>(pa.devicePointer);
-            to_caller = true;
-        } else {
-            cudaGetLastError();
-        }
-    }
+    CellRecord* caller_alias = direct ? static_cast<CellRecord*>(pinned_alias(out_host)) : nullptr;
+    CellRecord* rec_target = caller_alias ? caller_alias : direct ? e->h_records.p : e->d_records.p;
     auto& g = e->hg;
-    const bool same = g.seen && g.n_blocks == n_blocks && g.M == M && g.P == P && g.D == D && g.kind == kind &&
-                      g.iq_dev == e->iq_own.p && g.rec_dev == e->d_records.p && g.iq_stage == e->h_iq.p &&
-                      g.rec_stage == e->h_records.p && g.spec == e->spec.p && g.stream == e->stream &&
-                      g.d_dop == e->d_doppler.p && g.d_prn == e->d_ints.p && g.crep == e->crep.p &&
-                      g.rec_target == rec_target &&
-                      memcmp(g.dop.data(), dop, sizeof(double) * D) == 0 && memcmp(g.prn.data(), prn_idx, sizeof(int) * P) == 0;
+    // what a graph captured now would bake in (a first eager call may still grow the spectra scratch)
+    auto key_now = [&] {
+        return gb200_engine::HostGraph::Key{n_blocks, M, P, D, kind, e->iq_own.p, e->d_records.p, e->h_iq.p, e->h_records.p,
+                                            e->spec.p, e->d_doppler.p, e->d_ints.p, e->crep.p, rec_target, e->stream};
+    };
+    const bool same = g.seen && g.key == key_now() && memcmp(g.dop.data(), dop, sizeof(double) * D) == 0 &&
+                      memcmp(g.prn.data(), prn_idx, sizeof(int) * P) == 0;
     auto enqueue = [&]() -> int {
         GB_CUDA(e, cudaMemcpyAsync(e->iq_own.p, h2d_src, n_iq * sizeof(float2), cudaMemcpyHostToDevice, e->stream));
-        int rc = run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, rec_target);
-        if (rc) return rc;
+        GB_TRY(run_grid(e, n_blocks, M, prn_idx, P, dop, D, kind, rec_target));
         if (!direct)
             GB_CUDA(e, cudaMemcpyAsync(e->h_records.p, e->d_records.p, n_rec * sizeof(CellRecord), cudaMemcpyDeviceToHost, e->stream));
         return GB200_OK;
     };
     if (eager_src) {
-        int rc = enqueue();
-        if (rc) return rc;
+        GB_TRY(enqueue());
     } else if (same && g.exec) {
         GB_CUDA(e, cudaGraphLaunch(g.exec, e->stream));
         e->launches += 2;
@@ -919,31 +900,16 @@ int gb200_acquire_grid_host(gb200_engine* e, const float* iq_host, int n_blocks,
             if (g.exec) cudaGraphExecDestroy(g.exec);
             g.exec = nullptr;
         }
-        int rc = enqueue();
-        if (rc) return rc;
+        GB_TRY(enqueue());
         if (!same) {
-            g.n_blocks = n_blocks;
-            g.M = M;
-            g.P = P;
-            g.D = D;
-            g.kind = kind;
+            g.key = key_now();
             g.dop.assign(dop, dop + D);
             g.prn.assign(prn_idx, prn_idx + P);
-            g.iq_dev = e->iq_own.p;
-            g.rec_dev = e->d_records.p;
-            g.iq_stage = e->h_iq.p;
-            g.rec_stage = e->h_records.p;
-            g.spec = e->spec.p;
-            g.d_dop = e->d_doppler.p;
-            g.d_prn = e->d_ints.p;
-            g.crep = e->crep.p;
-            g.rec_target = rec_target;
-            g.stream = e->stream;
             g.seen = 1;
         }
     }
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    if (!to_caller) memcpy(out_host, e->h_records.p, n_rec * sizeof(CellRecord));
+    if (!caller_alias) memcpy(out_host, e->h_records.p, n_rec * sizeof(CellRecord));
     return GB200_OK;
 }
 
@@ -978,8 +944,6 @@ int gb200_ring_destroy(gb200_ring* r) {
         e->iq = nullptr;
         e->iq_samples = 0;
     }
-    r->buf.release();
-    r->h_stage.release();
     delete r;
     return GB200_OK;
 }
@@ -991,13 +955,8 @@ int gb200_ring_append(gb200_ring* r, const float* iq_host, int n_ms) {
     if (n_ms > r->capacity) GB_FAIL(e, GB200_EINVAL, "%d ms do not fit a ring of %d ms", n_ms, r->capacity);
     GB_CUDA(e, cudaSetDevice(e->device));
     const size_t N = static_cast<size_t>(e->N);
-    const float2* src = reinterpret_cast<const float2*>(iq_host);
-    if (!is_pinned_host(iq_host)) {
-        GB_CUDA(e, cudaStreamSynchronize(e->stream));  // staging buffer may still be in flight
-        GB_CUDA(e, r->h_stage.ensure(N * n_ms));
-        memcpy(r->h_stage.p, iq_host, N * n_ms * sizeof(float2));
-        src = r->h_stage.p;
-    }
+    const float2* src = nullptr;
+    GB_TRY(pinned_source(e, r->h_stage, iq_host, N * n_ms, &src));
     int done = 0;
     while (done < n_ms) {
         const int slot = static_cast<int>((r->appended + done) % r->capacity);
@@ -1038,8 +997,7 @@ int gb200_acquire_cells(gb200_engine* e, int n_cells, const int32_t* prn_idx, co
     GB_CUDA(e, cudaSetDevice(e->device));
     if (n_cells < 1) GB_FAIL(e, GB200_EINVAL, "empty cell list");
     GB_CUDA(e, e->d_records.ensure(n_cells));
-    int rc = run_cells(e, n_cells, prn_idx, dop, probe, n_ms, kind, e->d_records.p, nullptr);
-    if (rc) return rc;
+    GB_TRY(run_cells(e, n_cells, prn_idx, dop, probe, n_ms, kind, e->d_records.p, nullptr));
     return fetch_records(e, n_cells, out_host);
 }
 
@@ -1048,28 +1006,19 @@ int gb200_correlation_profile(gb200_engine* e, int prn, double dop, int n_ms, in
     if (!out_host) GB_FAIL(e, GB200_EINVAL, "null output");
     GB_CUDA(e, cudaSetDevice(e->device));
     const size_t nf = static_cast<size_t>(e->N) * (kind == GB200_COHERENT ? 2 : 1);
-    GB_CUDA(e, e->d_profile.ensure(nf));
-    GB_CUDA(e, e->h_profile.ensure(nf));
+    GB_CUDA(e, ensure_staging(e->d_profile, e->h_profile, nf));
     GB_CUDA(e, e->d_records.ensure(1));
     const int32_t p = prn;
-    int rc = run_cells(e, 1, &p, &dop, nullptr, n_ms, kind, e->d_records.p, e->d_profile.p);
-    if (rc) return rc;
-    GB_CUDA(e, cudaMemcpyAsync(e->h_profile.p, e->d_profile.p, nf * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-    GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->h_profile.p, nf * sizeof(float));
-    return GB200_OK;
+    GB_TRY(run_cells(e, 1, &p, &dop, nullptr, n_ms, kind, e->d_records.p, e->d_profile.p));
+    return download(e, out_host, e->h_profile, e->d_profile.p, nf);
 }
 
 int gb200_correlation_profile_replica(gb200_engine* e, const float* replica_host, double dop, int n_ms, int kind,
                                       float* out_host) {
     if (!e) return GB200_EINVAL;
     if (!replica_host || !out_host) GB_FAIL(e, GB200_EINVAL, "null buffer");
-    if (kind != GB200_COHERENT && kind != GB200_NON_COHERENT) GB_FAIL(e, GB200_EINVAL, "Unexpected integration type");
-    if (!e->iq) GB_FAIL(e, GB200_ESTATE, "no IQ loaded (gb200_upload_iq / gb200_bind_iq_device)");
-    if (n_ms < 1) GB_FAIL(e, GB200_EINVAL, "need at least one whole millisecond of samples");
-    if (static_cast<int64_t>(n_ms) * e->N > e->iq_samples)
-        GB_FAIL(e, GB200_EINVAL, "need %lld samples, %lld loaded", static_cast<long long>(n_ms) * e->N,
-                static_cast<long long>(e->iq_samples));
+    GB_TRY(check_common(e, n_ms, kind, false));
+    GB_TRY(check_samples(e, n_ms));
     GB_CUDA(e, cudaSetDevice(e->device));
     const size_t nf = static_cast<size_t>(e->N) * (kind == GB200_COHERENT ? 2 : 1);
     GB_CUDA(e, cudaStreamSynchronize(e->stream));  // staging buffers may still be in flight
@@ -1081,10 +1030,7 @@ int gb200_correlation_profile_replica(gb200_engine* e, const float* replica_host
     GB_CUDA(e, launch_correlate_generic(e->iq, e->d_replica.p, e->N, n_ms, dop, 1.0 / static_cast<double>(e->fs), kind,
                                         e->d_profile.p, e->stream));
     e->launches++;
-    GB_CUDA(e, cudaMemcpyAsync(e->h_profile.p, e->d_profile.p, nf * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-    GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->h_profile.p, nf * sizeof(float));
-    return GB200_OK;
+    return download(e, out_host, e->h_profile, e->d_profile.p, nf);
 }
 
 int gb200_enable_kernel_timing(gb200_engine* e, int on) {
@@ -1120,21 +1066,15 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
     if (!e) return GB200_EINVAL;
     if (!out_host) GB_FAIL(e, GB200_EINVAL, "null output");
     GB_CUDA(e, cudaSetDevice(e->device));
-    int rc = check_common(e, n_ms, GB200_NON_COHERENT);
-    if (rc) return rc;
+    GB_TRY(check_common(e, n_ms, GB200_NON_COHERENT));
     if (n_sv < 1 || !prn_idx) GB_FAIL(e, GB200_EINVAL, "no satellites to search for");
-    if (static_cast<int64_t>(n_ms) * e->N > e->iq_samples)
-        GB_FAIL(e, GB200_EINVAL, "need %lld samples, %lld loaded", static_cast<long long>(n_ms) * e->N,
-                static_cast<long long>(e->iq_samples));
-    for (int i = 0; i < n_sv; ++i)
-        if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
+    GB_TRY(check_samples(e, n_ms));
+    GB_TRY(check_prns(e, prn_idx, n_sv));
 
     const int MAXB = kRefineMaxBins;
     const int n_cells = n_sv * MAXB;
-    const int nw = pick_w2048(e, n_ms, GB200_NON_COHERENT, false);
-    const int np = nw ? nw : pick_np(e, n_ms, GB200_NON_COHERENT, false);
-    const int rsplit = pick_rsplit(e, np, n_cells);
-    const int cpg = np / rsplit;
+    const CorrPlan plan = plan_correlate(e, n_ms, GB200_NON_COHERENT, false, n_cells);
+    const int cpg = plan.cpg;
     const int gps = (MAXB + cpg - 1) / cpg;  // groups per satellite
     const size_t unit = unit_floats2(e, n_ms);
     int sv_per_chunk = static_cast<int>(std::max<size_t>(1, e->spec_budget_bytes / (unit * sizeof(float2) * MAXB)));
@@ -1146,10 +1086,8 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
     const int ng = n_sv * gps;
     const size_t n_ints = static_cast<size_t>(2) * n_cells + 3 * ng + 6 * n_sv;
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    GB_CUDA(e, e->r_ints.ensure(n_ints));
-    GB_CUDA(e, e->rh_ints.ensure(n_ints));
-    int* hi = e->rh_ints.p;
-    int* cell_u = hi;
+    GB_CUDA(e, ensure_staging(e->r_ints, e->rh_ints, n_ints));
+    int* cell_u = e->rh_ints.p;
     int* cell_out = cell_u + n_cells;
     int* g_first = cell_out + n_cells;
     int* g_count = g_first + ng;
@@ -1176,73 +1114,28 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
         cg_prn[sv] = prn_idx[sv];
     }
     int* di = e->r_ints.p;
-    GB_CUDA(e, cudaMemcpyAsync(di, hi, sizeof(int) * (n_ints - n_sv), cudaMemcpyHostToDevice, e->stream));
+    GB_CUDA(e, cudaMemcpyAsync(di, cell_u, sizeof(int) * (n_ints - n_sv), cudaMemcpyHostToDevice, e->stream));
     int* d_probe = di + (n_ints - n_sv);
 
     GB_CUDA(e, e->r_state.ensure(n_sv));
     GB_CUDA(e, e->r_doppler.ensure(static_cast<size_t>(n_cells) + n_sv));
     GB_CUDA(e, e->r_records.ensure(static_cast<size_t>(n_cells) + n_sv));
-    GB_CUDA(e, e->r_results.ensure(n_sv));
-    GB_CUDA(e, e->rh_results.ensure(n_sv));
+    GB_CUDA(e, ensure_staging(e->r_results, e->rh_results, n_sv));
     GB_CUDA(e, e->spec.ensure(unit * std::max(sv_per_chunk * MAXB, n_sv)));
     double* d_coh_doppler = e->r_doppler.p + n_cells;
     CellRecord* d_coh_records = e->r_records.p + n_cells;
 
-    auto spectra = [&](const double* dop, int n_units) -> cudaError_t {
-        SpectraArgs sa{};
-        sa.iq = e->iq;
-        sa.doppler = dop;
-        sa.spec = e->spec.p;
-        sa.tw1 = e->tw1.p;
-        sa.tw2 = e->tw2.p;
-        sa.block_stride = 0;
-        sa.inv_fs = 1.0 / static_cast<double>(e->fs);
-        sa.N = e->N;
-        sa.s = e->s;
-        sa.M = n_ms;
-        sa.n_doppler = n_units;
-        sa.n_units = n_units;
-        TimedLaunch tl(e, 0);
-        e->launches++;
-        return launch_doppler_spectra(sa, e->stream);
-    };
-    CorrelateArgs base{};
-    base.spec = e->spec.p;
-    base.crep = e->crep.p;
-    base.tw1 = e->tw1.p;
-    base.tw2 = e->tw2.p;
-    base.profile = nullptr;
-    base.N = e->N;
-    base.s = e->s;
-    base.M = n_ms;
-    base.rsplit = rsplit;
-    base.grid_mode = 0;
-
     // Every (satellite, bin) cell of a refinement pass has its own Doppler, so nothing is shared between PRNs: the
     // fused block-per-cell kernel does the same arithmetic without the spectra round trip through HBM.
     const bool use_fused = fused_supports(e->s) && e->detect_fused;
-    FusedArgs fbase{};
-    const int* d_cell_prn = nullptr;
     if (use_fused) {
-        if (!e->fused_configured) {
-            GB_CUDA(e, configure_fused_kernel());
-            e->fused_configured = true;
-        }
+        GB_CUDA(e, ensure_fused_configured(e));
         // [n_cells] replica row of every (satellite, bin) slot, then [n_sv] one per satellite for the coherent pass
-        GB_CUDA(e, e->r_cell_prn.ensure(static_cast<size_t>(n_cells) + n_sv));
-        GB_CUDA(e, e->rh_cell_prn.ensure(static_cast<size_t>(n_cells) + n_sv));
+        GB_CUDA(e, ensure_staging(e->r_cell_prn, e->rh_cell_prn, static_cast<size_t>(n_cells) + n_sv));
         for (int c = 0; c < n_cells; ++c) e->rh_cell_prn.p[c] = prn_idx[c / MAXB];
         for (int sv = 0; sv < n_sv; ++sv) e->rh_cell_prn.p[n_cells + sv] = prn_idx[sv];
         GB_CUDA(e, cudaMemcpyAsync(e->r_cell_prn.p, e->rh_cell_prn.p, sizeof(int) * (n_cells + n_sv), cudaMemcpyHostToDevice,
                                    e->stream));
-        d_cell_prn = e->r_cell_prn.p;
-        fbase.iq = e->iq;
-        fbase.crep = e->crep.p;
-        fbase.tw1 = e->tw1.p;
-        fbase.tw2 = e->tw2.p;
-        fbase.inv_fs = 1.0 / static_cast<double>(e->fs);
-        fbase.N = e->N;
-        fbase.M = n_ms;
     }
 
     GB_CUDA(e, launch_refine_init(n_sv, e->r_state.p, e->stream));
@@ -1252,38 +1145,20 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
         e->launches++;
         if (use_fused) {
             // one launch per pass: a CTA per (satellite, bin) slot, no spectra scratch
-            FusedArgs fa = fbase;
-            fa.doppler = e->r_doppler.p;
-            fa.prn = d_cell_prn;
-            fa.probe = nullptr;
-            fa.records = e->r_records.p;
-            fa.n_cells = n_cells;
-            {
-                TimedLaunch tl(e, 1);
-                GB_CUDA(e, launch_acquire_fused(fa, e->s, GB200_NON_COHERENT, e->stream));
-            }
-            e->launches++;
+            GB_TRY(enqueue_fused(e, n_ms, GB200_NON_COHERENT, e->r_doppler.p, e->r_cell_prn.p, nullptr, e->r_records.p, n_cells));
         }
         for (int sv0 = 0; !use_fused && sv0 < n_sv; sv0 += sv_per_chunk) {
             const int nsv = std::min(sv_per_chunk, n_sv - sv0);
-            GB_CUDA(e, spectra(e->r_doppler.p + static_cast<size_t>(sv0) * MAXB, nsv * MAXB));
-            CorrelateArgs ca = base;
-            ca.records = e->r_records.p;
-            ca.kind = GB200_NON_COHERENT;
+            GB_TRY(enqueue_spectra(e, e->iq, 0, e->r_doppler.p + static_cast<size_t>(sv0) * MAXB, n_ms, nsv * MAXB, nsv * MAXB));
+            CorrelateArgs ca = correlate_args(e, n_ms, GB200_NON_COHERENT, e->r_records.p);
             ca.n_groups = nsv * gps;
             ca.cell_u = di;
             ca.cell_out = di + n_cells;
             ca.grp_first = di + 2 * n_cells + sv0 * gps;
             ca.grp_count = di + 2 * n_cells + ng + sv0 * gps;
             ca.grp_prn = di + 2 * n_cells + 2 * ng + sv0 * gps;
-            ca.cell_probe = nullptr;
             ca.cell_gate = e->r_doppler.p;
-            {
-                TimedLaunch tl(e, 1);
-                if (nw) GB_CUDA(e, launch_correlate_w2048(ca, nw, std::min(ca.n_groups, e->num_sms), e->stream));
-                else GB_CUDA(e, launch_correlate_cells(ca, np, std::min(ca.n_groups, e->num_sms), e->stream));
-            }
-            e->launches++;
+            GB_TRY(enqueue_correlate(e, plan, ca, std::min(ca.n_groups, e->num_sms)));
         }
         GB_CUDA(e, launch_refine_select(n_sv, e->N, e->r_records.p, e->r_doppler.p, e->r_state.p, e->stream));
         e->launches++;
@@ -1292,26 +1167,11 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
     GB_CUDA(e, launch_refine_coherent_plan(n_sv, e->r_state.p, d_coh_doppler, d_probe, e->stream));
     e->launches++;
     if (use_fused) {
-        FusedArgs fa = fbase;
-        fa.doppler = d_coh_doppler;
-        fa.prn = d_cell_prn + n_cells;
-        fa.probe = d_probe;
-        fa.records = d_coh_records;
-        fa.n_cells = n_sv;
-        {
-            TimedLaunch tl(e, 1);
-            GB_CUDA(e, launch_acquire_fused(fa, e->s, GB200_COHERENT, e->stream));
-        }
-        e->launches++;
+        GB_TRY(enqueue_fused(e, n_ms, GB200_COHERENT, d_coh_doppler, e->r_cell_prn.p + n_cells, d_probe, d_coh_records, n_sv));
     } else {
-        GB_CUDA(e, spectra(d_coh_doppler, n_sv));
-    }
-    if (!use_fused) {
+        GB_TRY(enqueue_spectra(e, e->iq, 0, d_coh_doppler, n_ms, n_sv, n_sv));
         const int* cbase = di + 2 * n_cells + 3 * ng;
-        CorrelateArgs ca = base;
-        ca.records = d_coh_records;
-        ca.kind = GB200_COHERENT;
-        ca.rsplit = pick_rsplit(e, 8, n_sv);  // the coherent pass always runs on the 8-pair build
+        CorrelateArgs ca = correlate_args(e, n_ms, GB200_COHERENT, d_coh_records);
         ca.n_groups = n_sv;
         ca.cell_u = cbase;
         ca.cell_out = cbase + n_sv;
@@ -1319,46 +1179,36 @@ int gb200_detect(gb200_engine* e, int n_sv, const int32_t* prn_idx, int n_ms, gb
         ca.grp_count = cbase + 3 * n_sv;
         ca.grp_prn = cbase + 4 * n_sv;
         ca.cell_probe = d_probe;
-        ca.cell_gate = nullptr;
-        TimedLaunch tl(e, 1);
-        GB_CUDA(e, launch_correlate_cells(ca, 8, std::min(n_sv, e->num_sms), e->stream));
-        e->launches++;
+        const int rsplit = pick_rsplit(e, 8, n_sv);  // the coherent pass always runs on the 8-pair build
+        GB_TRY(enqueue_correlate(e, CorrPlan{0, 8, rsplit, 8 / rsplit}, ca, std::min(n_sv, e->num_sms)));
     }
     GB_CUDA(e, launch_refine_finalize(n_sv, e->r_state.p, d_coh_records, e->r_results.p, e->stream));
     e->launches++;
-    GB_CUDA(e, cudaMemcpyAsync(e->rh_results.p, e->r_results.p, sizeof(RefineResult) * n_sv, cudaMemcpyDeviceToHost, e->stream));
-    GB_CUDA(e, cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->rh_results.p, sizeof(RefineResult) * n_sv);
-    return GB200_OK;
+    return download(e, out_host, e->rh_results, e->r_results.p, n_sv);
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // tracking
 // ---------------------------------------------------------------------------------------------------------
-int gb200_tracker_create(gb200_engine* e, int n_channels, const int32_t* prn_idx, const double* doppler_hz,
-                         const double* carrier_phase, const int32_t* code_phase, gb200_tracker** out) {
-    if (!e) return GB200_EINVAL;
-    if (!out) GB_FAIL(e, GB200_EINVAL, "null output");
-    *out = nullptr;
-    if (n_channels < 1 || !prn_idx || !doppler_hz || !carrier_phase || !code_phase) GB_FAIL(e, GB200_EINVAL, "no channels");
+// Both tracker constructors: n channel slots whose device states are uploaded from init with every slot seeded
+// (gb200_tracker_create, whose PRN rows prn_idx are checked first) or, with init null, zeroed and unseeded (a pool).
+static int new_tracker(gb200_engine* e, int n, const int32_t* prn_idx, const TrackState* init, gb200_tracker** out) {
     if (e->s != 2 && e->s != 4) GB_FAIL(e, GB200_EINVAL, "tracking needs 2046 or 4092 samples per ms (reference tracker.py:301 hard-wires 2046)");
-    if (e->n_prn == 0) GB_FAIL(e, GB200_ESTATE, "no PRN replicas loaded (gb200_set_replicas)");
-    for (int c = 0; c < n_channels; ++c)
-        if (prn_idx[c] < 0 || prn_idx[c] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[c]);
+    if (init) {
+        if (e->n_prn == 0) GB_FAIL(e, GB200_ESTATE, "no PRN replicas loaded (gb200_set_replicas)");
+        GB_TRY(check_prns(e, prn_idx, n));
+    }
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, configure_track_kernel());
     gb200_tracker* t = new gb200_tracker;
     t->e = e;
-    t->n_channels = n_channels;
-    t->seeded.assign(n_channels, 1);
-    t->undo_ok.assign(n_channels, 0);
-    std::vector<TrackState> init(n_channels);
-    for (int c = 0; c < n_channels; ++c) {
-        memset(&init[c], 0, sizeof(TrackState));
-        track_state_init(init[c], prn_idx[c], doppler_hz[c], carrier_phase[c], code_phase[c]);
-    }
-    cudaError_t ce = t->states.ensure(n_channels);
-    if (ce == cudaSuccess) ce = cudaMemcpy(t->states.p, init.data(), sizeof(TrackState) * n_channels, cudaMemcpyHostToDevice);
+    t->n_channels = n;
+    t->seeded.assign(n, init ? 1 : 0);
+    t->undo_ok.assign(n, 0);
+    const size_t bytes = sizeof(TrackState) * n;
+    cudaError_t ce = t->states.ensure(n);
+    if (ce == cudaSuccess)
+        ce = init ? cudaMemcpy(t->states.p, init, bytes, cudaMemcpyHostToDevice) : cudaMemset(t->states.p, 0, bytes);
     if (ce != cudaSuccess) {
         delete t;
         cudaGetLastError();
@@ -1368,27 +1218,24 @@ int gb200_tracker_create(gb200_engine* e, int n_channels, const int32_t* prn_idx
     return GB200_OK;
 }
 
+int gb200_tracker_create(gb200_engine* e, int n_channels, const int32_t* prn_idx, const double* doppler_hz,
+                         const double* carrier_phase, const int32_t* code_phase, gb200_tracker** out) {
+    if (!e) return GB200_EINVAL;
+    if (!out) GB_FAIL(e, GB200_EINVAL, "null output");
+    *out = nullptr;
+    if (n_channels < 1 || !prn_idx || !doppler_hz || !carrier_phase || !code_phase) GB_FAIL(e, GB200_EINVAL, "no channels");
+    std::vector<TrackState> init(n_channels);
+    for (int c = 0; c < n_channels; ++c) {
+        memset(&init[c], 0, sizeof(TrackState));
+        track_state_init(init[c], prn_idx[c], doppler_hz[c], carrier_phase[c], code_phase[c]);
+    }
+    return new_tracker(e, n_channels, prn_idx, init.data(), out);
+}
+
 int gb200_tracker_destroy(gb200_tracker* t) {
     if (!t) return GB200_OK;
     cudaSetDevice(t->e->device);
     cudaStreamSynchronize(t->e->stream);
-    t->states.release();
-    t->shadow.release();
-    t->d_sel.release();
-    t->h_sel.release();
-    t->d_out.release();
-    t->d_times.release();
-    t->d_prof.release();
-    t->h_out.release();
-    t->h_times.release();
-    t->h_prof.release();
-    t->bit_states.release();
-    t->d_events.release();
-    t->d_counts.release();
-    t->d_bit_times.release();
-    t->h_events.release();
-    t->h_counts.release();
-    t->h_bit_times.release();
     delete t;
     return GB200_OK;
 }
@@ -1400,13 +1247,11 @@ static int tracker_launch(gb200_tracker* t, int n_sel, const int32_t* sel, int n
     gb200_engine* e = t->e;
     if (n_ms < 1 || !start_times) GB_FAIL(e, GB200_EINVAL, "need at least one whole millisecond of samples");
     if (!e->iq) GB_FAIL(e, GB200_ESTATE, "no IQ loaded (gb200_upload_iq / gb200_bind_iq_device)");
-    if (static_cast<int64_t>(n_ms) * e->N > e->iq_samples)
-        GB_FAIL(e, GB200_EINVAL, "need %lld samples, %lld loaded", static_cast<long long>(n_ms) * e->N,
-                static_cast<long long>(e->iq_samples));
+    GB_TRY(check_samples(e, n_ms));
     if (reinterpret_cast<uintptr_t>(e->iq) % 16 != 0) GB_FAIL(e, GB200_EINVAL, "IQ buffer must be 16-byte aligned for tracking");
     if (sel) {
         for (int i = 0; i < n_sel; ++i) {
-            if (sel[i] < 0 || sel[i] >= t->n_channels) GB_FAIL(e, GB200_EINVAL, "channel %d out of range", sel[i]);
+            GB_TRY(check_channel(t, sel[i]));
             if (!t->seeded[sel[i]]) GB_FAIL(e, GB200_ESTATE, "channel %d was never seeded (gb200_tracker_reset_channel)", sel[i]);
             for (int j = 0; j < i; ++j)
                 if (sel[j] == sel[i]) GB_FAIL(e, GB200_EINVAL, "channel %d listed twice", sel[i]);
@@ -1421,20 +1266,14 @@ static int tracker_launch(gb200_tracker* t, int n_sel, const int32_t* sel, int n
         a.t0_single = start_times[0];
     } else {
         GB_CUDA(e, cudaStreamSynchronize(e->stream));  // h_times may still be in flight
-        GB_CUDA(e, t->d_times.ensure(n_ms));
-        GB_CUDA(e, t->h_times.ensure(n_ms));
-        memcpy(t->h_times.p, start_times, sizeof(double) * n_ms);
-        GB_CUDA(e, cudaMemcpyAsync(t->d_times.p, t->h_times.p, sizeof(double) * n_ms, cudaMemcpyHostToDevice, e->stream));
+        GB_TRY(stage_upload(e, t->d_times, t->h_times, start_times, n_ms));
         a.start_times = t->d_times.p;
     }
     if (sel) {
         const bool cached = static_cast<int>(t->sel_cache.size()) == n_sel && memcmp(t->sel_cache.data(), sel, sizeof(int) * n_sel) == 0;
         if (!cached) {  // the subset rarely changes between calls: upload it only when it did
             GB_CUDA(e, cudaStreamSynchronize(e->stream));
-            GB_CUDA(e, t->d_sel.ensure(n_sel));
-            GB_CUDA(e, t->h_sel.ensure(n_sel));
-            memcpy(t->h_sel.p, sel, sizeof(int) * n_sel);
-            GB_CUDA(e, cudaMemcpyAsync(t->d_sel.p, t->h_sel.p, sizeof(int) * n_sel, cudaMemcpyHostToDevice, e->stream));
+            GB_TRY(stage_upload(e, t->d_sel, t->h_sel, sel, n_sel));
             t->sel_cache.assign(sel, sel + n_sel);
         }
         a.channel_idx = t->d_sel.p;
@@ -1478,16 +1317,11 @@ static int tracker_process_host(gb200_tracker* t, int n_sel, const int32_t* sel,
     if (n_ms < 1) GB_FAIL(e, GB200_EINVAL, "need at least one whole millisecond of samples");
     if (n_sel < 1) GB_FAIL(e, GB200_EINVAL, "no channels");
     const size_t n = static_cast<size_t>(n_sel) * n_ms;
-    GB_CUDA(e, t->d_out.ensure(n));
-    GB_CUDA(e, t->h_out.ensure(n));
+    GB_CUDA(e, ensure_staging(t->d_out, t->h_out, n));
     const size_t np = profiles_host ? n * e->N : 0;
-    if (np) {
-        GB_CUDA(e, t->d_prof.ensure(np));
-        GB_CUDA(e, t->h_prof.ensure(np));
-    }
+    if (np) GB_CUDA(e, ensure_staging(t->d_prof, t->h_prof, np));
     t->last_n_ms = 0;
-    int rc = tracker_launch(t, n_sel, sel, n_ms, start_times, t->d_out.p, np ? t->d_prof.p : nullptr, keep_undo);
-    if (rc) return rc;
+    GB_TRY(tracker_launch(t, n_sel, sel, n_ms, start_times, t->d_out.p, np ? t->d_prof.p : nullptr, keep_undo));
     if (!sel) t->last_n_ms = n_ms;  // gb200_tracker_integrate_bits reads [channel][n_ms] of the whole bank
     GB_CUDA(e, cudaMemcpyAsync(t->h_out.p, t->d_out.p, n * sizeof(TrackMsRecord), cudaMemcpyDeviceToHost, e->stream));
     if (np) GB_CUDA(e, cudaMemcpyAsync(t->h_prof.p, t->d_prof.p, np * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
@@ -1513,7 +1347,7 @@ int gb200_tracker_process_channels(gb200_tracker* t, int n_sel, const int32_t* c
 int gb200_tracker_undo_channel(gb200_tracker* t, int channel) {
     if (!t) return GB200_EINVAL;
     gb200_engine* e = t->e;
-    if (channel < 0 || channel >= t->n_channels) GB_FAIL(e, GB200_EINVAL, "channel %d out of range", channel);
+    GB_TRY(check_channel(t, channel));
     if (!t->undo_ok[channel]) GB_FAIL(e, GB200_ESTATE, "channel %d has no kept state to go back to", channel);
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, cudaMemcpyAsync(t->states.p + channel, t->shadow.p + channel, sizeof(TrackState), cudaMemcpyDeviceToDevice, e->stream));
@@ -1526,31 +1360,15 @@ int gb200_tracker_create_pool(gb200_engine* e, int capacity, gb200_tracker** out
     if (!out) GB_FAIL(e, GB200_EINVAL, "null output");
     *out = nullptr;
     if (capacity < 1) GB_FAIL(e, GB200_EINVAL, "no channels");
-    if (e->s != 2 && e->s != 4) GB_FAIL(e, GB200_EINVAL, "tracking needs 2046 or 4092 samples per ms (reference tracker.py:301 hard-wires 2046)");
-    GB_CUDA(e, cudaSetDevice(e->device));
-    GB_CUDA(e, configure_track_kernel());
-    gb200_tracker* t = new gb200_tracker;
-    t->e = e;
-    t->n_channels = capacity;
-    t->seeded.assign(capacity, 0);
-    t->undo_ok.assign(capacity, 0);
-    cudaError_t ce = t->states.ensure(capacity);
-    if (ce == cudaSuccess) ce = cudaMemset(t->states.p, 0, sizeof(TrackState) * capacity);
-    if (ce != cudaSuccess) {
-        delete t;
-        cudaGetLastError();
-        GB_FAIL(e, GB200_ECUDA, "tracker state allocation failed: %s", cudaGetErrorString(ce));
-    }
-    *out = t;
-    return GB200_OK;
+    return new_tracker(e, capacity, nullptr, nullptr, out);
 }
 
 int gb200_tracker_reset_channel(gb200_tracker* t, int channel, int32_t prn_idx, double doppler_hz, double carrier_phase,
                                 int32_t code_phase) {
     if (!t) return GB200_EINVAL;
     gb200_engine* e = t->e;
-    if (channel < 0 || channel >= t->n_channels) GB_FAIL(e, GB200_EINVAL, "channel %d out of range", channel);
-    if (prn_idx < 0 || prn_idx >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx);
+    GB_TRY(check_channel(t, channel));
+    GB_TRY(check_prns(e, &prn_idx, 1));
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
     std::vector<TrackState> init(1);
@@ -1566,7 +1384,7 @@ int gb200_tracker_get_state(gb200_tracker* t, int channel, double* doppler_hz, d
                             int32_t* code_phase, int32_t* lost) {
     if (!t) return GB200_EINVAL;
     gb200_engine* e = t->e;
-    if (channel < 0 || channel >= t->n_channels) GB_FAIL(e, GB200_EINVAL, "channel %d out of range", channel);
+    GB_TRY(check_channel(t, channel));
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
     TrackState st;
@@ -1583,7 +1401,7 @@ int gb200_tracker_set_state(gb200_tracker* t, int channel, double doppler_hz, do
                             int32_t code_phase) {
     if (!t) return GB200_EINVAL;
     gb200_engine* e = t->e;
-    if (channel < 0 || channel >= t->n_channels) GB_FAIL(e, GB200_EINVAL, "channel %d out of range", channel);
+    GB_TRY(check_channel(t, channel));
     GB_CUDA(e, cudaSetDevice(e->device));
     GB_CUDA(e, cudaStreamSynchronize(e->stream));
     TrackState st;
@@ -1621,12 +1439,9 @@ int gb200_tracker_integrate_bits(gb200_tracker* t, int n_ms, const double* start
         GB_CUDA(e, cudaMemcpy(t->bit_states.p, init.data(), sizeof(BitState) * nc, cudaMemcpyHostToDevice));
     }
     const size_t ne = static_cast<size_t>(nc) * max_events;
-    GB_CUDA(e, t->d_events.ensure(ne));
-    GB_CUDA(e, t->h_events.ensure(ne));
-    GB_CUDA(e, t->d_counts.ensure(nc));
-    GB_CUDA(e, t->h_counts.ensure(nc));
-    GB_CUDA(e, t->d_bit_times.ensure(2 * static_cast<size_t>(n_ms)));
-    GB_CUDA(e, t->h_bit_times.ensure(2 * static_cast<size_t>(n_ms)));
+    GB_CUDA(e, ensure_staging(t->d_events, t->h_events, ne));
+    GB_CUDA(e, ensure_staging(t->d_counts, t->h_counts, nc));
+    GB_CUDA(e, ensure_staging(t->d_bit_times, t->h_bit_times, 2 * static_cast<size_t>(n_ms)));
     memcpy(t->h_bit_times.p, start_times, sizeof(double) * n_ms);
     memcpy(t->h_bit_times.p + n_ms, end_times, sizeof(double) * n_ms);
     GB_CUDA(e, cudaMemcpyAsync(t->d_bit_times.p, t->h_bit_times.p, 2 * sizeof(double) * n_ms, cudaMemcpyHostToDevice, e->stream));
@@ -1682,17 +1497,6 @@ int gb200_grid_stream_destroy(gb200_grid_stream* g) {
     cudaStreamSynchronize(g->e->stream);
     if (g->s_in) cudaStreamSynchronize(g->s_in);
     if (g->s_out) cudaStreamSynchronize(g->s_out);
-    for (auto& sl : g->slots) {
-        sl.iq.release();
-        sl.rec.release();
-        sl.h_iq.release();
-        sl.h_rec.release();
-        if (sl.h2d) cudaEventDestroy(sl.h2d);
-        if (sl.done) cudaEventDestroy(sl.done);
-        if (sl.d2h) cudaEventDestroy(sl.d2h);
-    }
-    if (g->s_in) cudaStreamDestroy(g->s_in);
-    if (g->s_out) cudaStreamDestroy(g->s_out);
     delete g;
     return GB200_OK;
 }
@@ -1704,10 +1508,8 @@ int gb200_grid_stream_create(gb200_engine* e, int n_blocks, int M, const int32_t
     *out = nullptr;
     if (n_blocks < 1 || P < 1 || D < 1 || !prn_idx || !dop) GB_FAIL(e, GB200_EINVAL, "empty grid");
     if (depth < 1 || depth > 8) GB_FAIL(e, GB200_EINVAL, "depth must be 1..8");
-    int rc = check_common(e, M, kind);
-    if (rc) return rc;
-    for (int i = 0; i < P; ++i)
-        if (prn_idx[i] < 0 || prn_idx[i] >= e->n_prn) GB_FAIL(e, GB200_EINVAL, "prn index %d out of range", prn_idx[i]);
+    GB_TRY(check_common(e, M, kind));
+    GB_TRY(check_prns(e, prn_idx, P));
     GB_CUDA(e, cudaSetDevice(e->device));
     gb200_grid_stream* g = new gb200_grid_stream;
     g->e = e;
@@ -1719,16 +1521,15 @@ int gb200_grid_stream_create(gb200_engine* e, int n_blocks, int M, const int32_t
     g->depth = depth;
     g->prn.assign(prn_idx, prn_idx + P);
     g->dop.assign(dop, dop + D);
-    g->slots.resize(depth);
+    g->slots = std::vector<gb200_grid_stream::Slot>(depth);
     const size_t n_iq = static_cast<size_t>(n_blocks) * M * e->N, n_rec = static_cast<size_t>(n_blocks) * P * D;
     cudaError_t ce = cudaStreamCreateWithFlags(&g->s_in, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&g->s_out, cudaStreamNonBlocking);
     for (auto& sl : g->slots) {
         if (ce == cudaSuccess) ce = sl.iq.ensure(n_iq);
         if (ce == cudaSuccess) ce = sl.rec.ensure(n_rec);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&sl.h2d, cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&sl.d2h, cudaEventDisableTiming);
+        for (cudaEvent_t* ev : {&sl.h2d, &sl.done, &sl.d2h})
+            if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
     }
     if (ce != cudaSuccess) {
         gb200_grid_stream_destroy(g);
@@ -1749,21 +1550,20 @@ int gb200_grid_stream_submit(gb200_grid_stream* g, const float* iq_host, gb200_c
     const size_t n_iq = static_cast<size_t>(g->n_blocks) * g->M * e->N, n_rec = static_cast<size_t>(g->n_blocks) * g->P * g->D;
     // the slot's previous batch was collected, so its device buffers and staging are free
     const void* src = iq_host;
-    if (!is_pinned_host(iq_host)) {
+    if (!pinned_alias(iq_host)) {
         GB_CUDA(e, sl.h_iq.ensure(n_iq));
         memcpy(sl.h_iq.p, iq_host, n_iq * sizeof(float2));
         src = sl.h_iq.p;
     }
     sl.out = out_host;
-    sl.staged_out = !is_pinned_host(out_host);
+    sl.staged_out = !pinned_alias(out_host);
     if (sl.staged_out) GB_CUDA(e, sl.h_rec.ensure(n_rec));
     GB_CUDA(e, cudaMemcpyAsync(sl.iq.p, src, n_iq * sizeof(float2), cudaMemcpyHostToDevice, g->s_in));
     GB_CUDA(e, cudaEventRecord(sl.h2d, g->s_in));
     GB_CUDA(e, cudaStreamWaitEvent(e->stream, sl.h2d, 0));
     e->iq = sl.iq.p;
     e->iq_samples = static_cast<int64_t>(n_iq);
-    int rc = run_grid(e, g->n_blocks, g->M, g->prn.data(), g->P, g->dop.data(), g->D, g->kind, sl.rec.p);
-    if (rc) return rc;
+    GB_TRY(run_grid(e, g->n_blocks, g->M, g->prn.data(), g->P, g->dop.data(), g->D, g->kind, sl.rec.p));
     GB_CUDA(e, cudaEventRecord(sl.done, e->stream));
     GB_CUDA(e, cudaStreamWaitEvent(g->s_out, sl.done, 0));
     GB_CUDA(e, cudaMemcpyAsync(sl.staged_out ? reinterpret_cast<gb200_cell_record*>(sl.h_rec.p) : out_host, sl.rec.p,
