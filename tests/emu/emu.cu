@@ -67,22 +67,17 @@ void emu_replica_spectrum(const uint8_t* chips, float2* crep) {
     }
 }
 
-// Full per-cell pipeline.  iq: complex64[n_ms*N]; out: float[N] (non-coherent) or float2[N] (coherent).
-// kind: 1 coherent, 2 non-coherent (utils.py:23-25).
-void emu_cell_profile(const float2* iq, int N, int n_ms, double fs, double doppler, const uint8_t* chips, int kind,
-                      float* out, CellRecord* rec_out) {
-    init_tables();
+}  // extern "C"
+
+// ---- doppler_spectra (mirrors k_doppler_spectra<S>: 256 "threads", carrier = coarse x fine table) ----
+// spec[i][r][half][1024] for the n_ms milliseconds of one Doppler bin
+static std::vector<float2> emu_spectra(const float2* iq, int N, int n_ms, double fs, double doppler) {
     const int s = N / kChips;
-    std::vector<float2> crep(2048);
-    emu_replica_spectrum(chips, crep.data());
-    std::vector<float2> tile(kTileF2), tileO(kTileF2);
+    std::vector<float2> tile(kTileF2);
     std::vector<float2> ypoly((size_t)s * kFft);
-    // spec[i][r][half][1024]
     std::vector<float2> spec((size_t)n_ms * s * 2 * kFft);
     WarpRegs* w = new WarpRegs;
-    WarpRegs* wo = new WarpRegs;
     const double inv_fs = 1.0 / fs;
-    // ---- doppler_spectra (mirrors k_doppler_spectra<S>: 256 "threads", carrier = coarse x fine table) ----
     for (int i = 0; i < n_ms; ++i) {
         float2 coarse[64], fine[256];
         for (int k = 0; k < (N + 255) / 256; ++k) coarse[k] = carrier_at(doppler, (double)(k * 256 + i * N), inv_fs);
@@ -116,6 +111,24 @@ void emu_cell_profile(const float2* iq, int N, int n_ms, double fs, double doppl
                 for (int lane = 0; lane < 32; ++lane) store_vec(w->x[lane], lane, dst);
             }
     }
+    delete w;
+    return spec;
+}
+
+extern "C" {
+
+// Full per-cell pipeline.  iq: complex64[n_ms*N]; out: float[N] (non-coherent) or float2[N] (coherent).
+// kind: 1 coherent, 2 non-coherent (utils.py:23-25).
+void emu_cell_profile(const float2* iq, int N, int n_ms, double fs, double doppler, const uint8_t* chips, int kind,
+                      float* out, CellRecord* rec_out) {
+    init_tables();
+    const int s = N / kChips;
+    std::vector<float2> crep(2048);
+    emu_replica_spectrum(chips, crep.data());
+    std::vector<float2> tile(kTileF2), tileO(kTileF2);
+    const std::vector<float2> spec = emu_spectra(iq, N, n_ms, fs, doppler);
+    WarpRegs* w = new WarpRegs;
+    WarpRegs* wo = new WarpRegs;
     // ---- correlate_cells ----
     if (kind == 2) memset(out, 0, sizeof(float) * N);
     else memset(out, 0, sizeof(float) * 2 * N);
@@ -191,6 +204,62 @@ void emu_cell_profile(const float2* iq, int N, int n_ms, double fs, double doppl
     }
     delete w;
     delete wo;
+}
+
+// One cell of k_correlate_w2048 (non-coherent): per polyphase branch r, one warp loads both half-spectra times the replica
+// spectrum, runs the pruned inverse FFT-2048 and accumulates |.| of its 32 lags q = lane + 32 k over the n_ms milliseconds;
+// the lags k < 16 and k >= 16 are reduced as the halves h = 0 / 1 of thread_peak16, and every thread's peaks are merged
+// into the cell record.  out: float[N], the accumulated profile at index s q + r.
+void emu_cell_record_w2048(const float2* iq, int N, int n_ms, double fs, double doppler, const uint8_t* chips, float* out,
+                           CellRecord* rec_out) {
+    init_tables();
+    const int s = N / kChips;
+    std::vector<float2> crep(2048);
+    emu_replica_spectrum(chips, crep.data());
+    std::vector<float2> tile(kTile64F2);
+    const std::vector<float2> spec = emu_spectra(iq, N, n_ms, fs, doppler);
+    static float acc[32][32];  // [lane][k]
+    Peak cell;
+    peak_init(cell);
+    for (int r = 0; r < s; ++r) {
+        memset(acc, 0, sizeof(acc));
+        for (int it = 0; it < n_ms; ++it) {
+            const float2* p = &spec[((size_t)it * s + r) * 2 * kFft];
+            for (int lane = 0; lane < 32; ++lane) {
+                float2 hx[32];
+                load_mul_vec(hx, lane, p, crep.data());  // even bins
+                w2048_phase1<0>(hx, lane, g_tw1.data(), tile.data());
+                load_mul_vec(hx, lane, p + kFft, crep.data() + kFft);  // odd bins
+                w2048_phase1<1>(hx, lane, g_tw1.data(), tile.data());
+            }
+            for (int lane = 0; lane < 32; ++lane) {
+                float2 x[64];
+                w2048_phase2(x, lane, tile.data());
+                for (int k = 0; k < 32; ++k) acc[lane][k] += gb_mag(x[k]);
+            }
+        }
+        for (int lane = 0; lane < 32; ++lane) {
+            for (int k = 0; k < 32; ++k) {
+                const int q = lane + 32 * k;
+                if (q < kChips) out[s * q + r] = acc[lane][k];
+            }
+            for (int hh = 0; hh < 2; ++hh) {
+                float v[16];
+                for (int jj = 0; jj < 16; ++jj) v[jj] = acc[lane][16 * hh + jj];
+                Peak t;
+                float fsum;
+                thread_peak16(v, lane, hh, s, r, t, fsum);
+                t.sum = (double)fsum;
+                peak_merge(cell, t);
+            }
+        }
+    }
+    rec_out->peak = cell.mx;
+    rec_out->argmax = cell.idx;
+    rec_out->sum = cell.sum;
+    rec_out->count = cell.cnt;
+    rec_out->probe_re = rec_out->probe_im = 0.f;
+    rec_out->pad_ = 0;
 }
 }
 

@@ -222,7 +222,7 @@ e.close()
 """
 
 
-@pytest.mark.parametrize("n, nb", [(2046, 20), (16368, 3)])
+@pytest.mark.parametrize("n, nb", [(2046, 20), (16368, 3), (12276, 3)])
 def test_l2_windows_leave_every_record_unchanged(engine_for, tmp_path, n, nb):
     """The one-warp kernel walks batches larger than L2 in windows of units (group order window / PRN / chunk, extra groups going
     round the CTAs).  That only reorders independent cells: with windows forced onto a small batch (a child process, the knobs
